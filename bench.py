@@ -5,6 +5,8 @@
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU algorithm
                                                            (oracle port; the reference itself
                                                            cannot be built here, DESIGN.md)
+  ... --dump-outputs DIR                                   also write the state and report of the
+                                                           last timed step as DIR/<name>.npy
 
 One "step" = one LM iteration = one call of OptimizeJointly(max_iteration_count=1): one H/b
 build over all observations, >= 1 Schur solve, >= 1 trial-cost pass (SURVEY.md 8d).
@@ -19,6 +21,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -26,9 +29,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 
 _emit = None
 BYTES_PER_OBS = {0: 720, 1: 1488, 3: 400}  # SURVEY.md 8(d): algorithmic bytes of the Jacobian kernel (C = 1)
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000  # --dump-outputs: data bytes written in all
 
 
 def _peaks():
@@ -81,21 +86,38 @@ class ClockSampler:
                 "reasons": sorted(self.reasons), "samples": len(sm)}
 
 
+def _workload_cache_path(args):
+    """File of this user's private workload cache for these arguments, or None when no private
+    directory is available. The name carries a digest of the generator's source, so a changed
+    generator never reads a workload an older one wrote."""
+    import hashlib
+    from camera_calibration_b200 import cabi, synthetic
+    h = hashlib.sha256()
+    for m in (synthetic, cabi):
+        with open(m.__file__, "rb") as f:
+            h.update(f.read())
+    d = os.path.join(tempfile.gettempdir(), f"b200ba_workload_{os.getuid()}")
+    try:
+        os.makedirs(d, mode=0o700, exist_ok=True)
+        st = os.stat(d)
+    except OSError:
+        return None
+    if st.st_uid != os.getuid() or st.st_mode & 0o077:
+        return None  # another user could write there, and the cache is unpickled
+    return os.path.join(d, f"c{args.config}_i{args.imagesets}_{h.hexdigest()[:16]}.pkl")
+
+
 def make_workload(args):
-    """Seeded synthetic problem; cached in /tmp so that several bench invocations on one box (and
-    the ranks of one torchrun) do not regenerate it -- generation is deterministic."""
+    """Seeded synthetic problem: the same arguments give the same inputs on every run. Cached in a
+    private temporary directory so that several bench invocations on one machine (and the ranks of
+    one torchrun) do not regenerate it -- generation is deterministic and takes about a minute."""
     import pickle
     from camera_calibration_b200 import synthetic
     kw = {}
     if args.imagesets:
         kw["n_imagesets"] = args.imagesets
-    cache = f"/tmp/b200ba_workload_c{args.config}_i{args.imagesets}_v2.pkl"
-    # a pre-generated copy shipped with the snapshot (workload_cache/, git-ignored: plain seeded synthetic data
-    # that every rank would otherwise regenerate for minutes of GPU-box time) takes precedence
-    shipped = os.path.join(ROOT, "workload_cache", os.path.basename(cache))
-    if os.path.exists(shipped):
-        cache = shipped
-    if os.path.exists(cache):
+    cache = _workload_cache_path(args)
+    if cache and os.path.exists(cache):
         try:
             d = pickle.load(open(cache, "rb"))
             from camera_calibration_b200.cabi import Camera, FlatProblem, FlatState
@@ -112,6 +134,8 @@ def make_workload(args):
         except Exception:
             pass
     sp = synthetic.make_problem(args.config, **kw)
+    if not cache:
+        return sp
     try:
         p = sp.problem
         st = lambda s: (s.points, s.rig_tr_global, s.camera_tr_rig, s.intrinsics,
@@ -119,8 +143,6 @@ def make_workload(args):
         d = dict(cams=[{k: getattr(c, k) for k, _ in c._fields_} for c in p.cameras], n_imagesets=p.n_imagesets,
                  n_points=p.n_points, oi=p.obs_imageset, oc=p.obs_camera, op=p.obs_point, oxy=p.obs_xy,
                  init=st(sp.init_state), gt=st(sp.gt_state), seed=sp.seed, info=sp.info, name=sp.name)
-        if cache.startswith(os.path.join(ROOT, "workload_cache")):
-            cache = f"/tmp/b200ba_workload_c{args.config}_i{args.imagesets}_v2.pkl"
         tmp = cache + f".{os.getpid()}"
         pickle.dump(d, open(tmp, "wb"))
         os.replace(tmp, cache)
@@ -202,7 +224,7 @@ class CpuTrajectory:
         # one thread per physical core, pinned and spread over the sockets (must be set before libgomp starts)
         os.environ.setdefault("OMP_PROC_BIND", "spread")
         os.environ.setdefault("OMP_PLACES", "cores")
-        self.threads = oracle.use_native(threads if threads > 0 else physical_cores())  # -march=native build made on THIS box
+        self.threads = oracle.use_native(threads if threads > 0 else physical_cores())  # -march=native, built for this CPU
         self.sp = sp
         self.opt = cabi.default_options(jacobian_mode=cabi.JACOBIAN_NUMERIC, max_iteration_count=1)
         # start state: the perturbed initial state with the projection cache warmed by one residual pass
@@ -227,6 +249,7 @@ class CpuTrajectory:
         t0 = time.perf_counter()
         self.state, rep = self.oracle.optimize(self.sp.problem, self.state, self.opt)
         dt = time.perf_counter() - t0
+        self.last = (self.state, rep)  # what this step returned, kept across a restart of the trajectory
         self.lam = rep.final_lambda
         self.breakdown["cost_and_jacobian_s"] += rep.cost_and_jacobian_evaluation_time
         self.breakdown["solve_s"] += rep.solve_time
@@ -238,6 +261,36 @@ class CpuTrajectory:
         else:
             self.last_cost = cost
         return dt, cost
+
+
+def dump_outputs(out_dir, state, rep):
+    """Writes what one timed step returns to its caller -- the state after the step and its report --
+    as float64 DIR/<name>.npy, so that two builds can be compared output for output on the same
+    inputs. last_projection (two values per observation) is the only array that grows with the
+    workload: when everything would exceed DUMP_LIMIT_BYTES, a fixed, seeded sample of its rows is
+    written instead, together with their indices (last_projection_rows)."""
+    arrays = {"points": state.points, "rig_tr_global": state.rig_tr_global, "camera_tr_rig": state.camera_tr_rig}
+    for c, a in enumerate(state.intrinsics):
+        arrays[f"intrinsics_{c}"] = a
+    for k in ("initial_cost", "final_cost", "final_lambda", "rmse", "n_valid", "n_invalid", "num_iterations_performed",
+              "performed_an_iteration"):
+        arrays[k] = getattr(rep, k)
+    arrays["trace_cost"], arrays["trace_lambda"], arrays["trace_attempts"] = rep.trace()
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    lp = np.asarray(state.last_projection, dtype=np.float64)
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values())
+    if lp.nbytes <= room:
+        arrays["last_projection"] = lp
+    else:
+        per_row = lp[0].nbytes + 8  # the row and its index
+        rows = np.sort(np.random.default_rng(0).choice(len(lp), room // per_row, replace=False))
+        arrays["last_projection"] = lp[rows]
+        arrays["last_projection_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+    return {"dir": out_dir, "arrays": sorted(arrays), "bytes": int(sum(a.nbytes for a in arrays.values())),
+            "last_projection_sampled": "last_projection_rows" in arrays}
 
 
 def cpu_baseline(sp, budget_s=60.0):
@@ -291,6 +344,8 @@ def run_reference(args):
         "breakdown_s_per_step": {k: v / done for k, v in traj.breakdown.items()},
         "steps_requested": K,
     }
+    if args.dump_outputs:
+        line["dump_outputs"] = dump_outputs(args.dump_outputs, *traj.last)
     _emit(line)
     return 0
 
@@ -403,9 +458,15 @@ def run_b200(args):
     con_flops = fac_flops = 0.0
     rmse = None
     restore_wall = 0.0
-    for _ in range(K):
+    dumped, dump_wall = None, 0.0
+    for i in range(K):
         opt.init_lambda = tr.lam
         rep = adj.optimize(opt)
+        if args.dump_outputs and i == K - 1:
+            # read back before the stop rule may restore the start state; untimed in `value` and in wall_ms
+            tw = time.perf_counter()
+            dumped = (adj.get_state(), rep)
+            dump_wall = time.perf_counter() - tw
         t = adj.timings()
         dev_ms += t.total_ms
         step_ms.append(t.total_ms)
@@ -430,7 +491,7 @@ def run_b200(args):
         if len(tr.lengths) != tr_before:
             restore_wall += time.perf_counter() - tw  # untimed in `value`; reported
     barrier()
-    wall_ms = 1e3 * (time.perf_counter() - t0 - restore_wall)
+    wall_ms = 1e3 * (time.perf_counter() - t0 - restore_wall - dump_wall)
     traj_lengths = list(tr.lengths)
 
     # ---- end to end: host buffers in, host buffers out, every step (b200ba_optimize_host) ---------------
@@ -544,6 +605,8 @@ def run_b200(args):
         line["dense_path"] = ("in-tree sm_100a kernels: DMMA contraction with scatter epilogue, blocked Cholesky on packed "
                               "panels (fused tile factor + inverse launch), packed triangular solves (ba_dense.cu, ba_tile.cuh)") if os.environ.get("B200BA_DENSE", "own") not in ("lib", "0") \
             else "cuBLAS dsyrk + cuSOLVER potrf / potrs (B200BA_DENSE=lib)"
+        if dumped is not None:
+            line["dump_outputs"] = dump_outputs(args.dump_outputs, *dumped)
     adj.close()
     adj = None
     if rank == 0:
@@ -585,7 +648,7 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed LM iterations (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", type=int, default=2)
@@ -595,7 +658,12 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=0, help="host threads of the CPU arm (0 = all cores)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-library-comparison", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state and report the last one returned as DIR/<name>.npy "
+                         "(float64, at most 64 MB; with several GPUs, rank 0's view: its shard of last_projection)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # Exactly ONE line goes to stdout (the JSON line): libraries (NCCL prints its version banner)
     # write to fd 1 directly, so fd 1 is pointed at stderr until the result is ready.
     sys.stdout.flush()

@@ -6,9 +6,12 @@ problem is handed to both sides.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -17,30 +20,35 @@ from camera_calibration_b200.cabi import Camera, FlatProblem, FlatState, Options
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_build", "libba_oracle.so")
-NATIVE_LIB_PATH = os.path.join(_HERE, "_build", "libba_oracle_native.so")
 _LIB = None
 _D = C.POINTER(C.c_double)
 _I32 = C.POINTER(C.c_int32)
 
 
 def build(force: bool = False, native: bool = False) -> str:
-    """Compile the oracle with the committed Makefile (g++, no dependencies). ``native=True``
-    builds the -march=native variant used by the timing legs of bench.py (on the box it runs on)."""
-    target = NATIVE_LIB_PATH if native else LIB_PATH
+    """Compile the oracle with the committed Makefile (g++, no dependencies) into oracle/_build/.
+    ``native=True`` builds the -march=native variant used by the timing legs of bench.py into a
+    fresh temporary directory instead: it must match the CPU it runs on, and the source tree may be
+    read-only at that point. The directory is removed when the process exits."""
+    if native:
+        out = tempfile.mkdtemp(prefix="ba_oracle_native_")
+        atexit.register(shutil.rmtree, out, True)
+        subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"BUILD={out}"], stdout=subprocess.DEVNULL)
+        return os.path.join(out, "libba_oracle_native.so")
+    target = os.path.join(_HERE, "_build", "libba_oracle.so")
     srcs = [os.path.join(_HERE, f) for f in ("ba_oracle.cc", "ba_oracle.h", "ba_dense_fast.h")] + [
         os.path.join(_HERE, "..", "include", "b200ba.h")]
     if force or not os.path.exists(target) or os.path.getmtime(target) < max(os.path.getmtime(f) for f in srcs):
-        cmd = ["make", "-C", _HERE, "-s"] + (["-B"] if force else []) + (["native"] if native else [])
+        cmd = ["make", "-C", _HERE, "-s"] + (["-B"] if force else [])
         subprocess.check_call(cmd, stdout=subprocess.DEVNULL)
     return target
 
 
 def use_native(threads: int = 0) -> int:
-    """Switch this process to the -march=native build (rebuilt here if stale) and set the host
-    thread count of the full-size kernels (0 = all cores). Returns the thread count in effect."""
+    """Switch this process to a -march=native build made on this machine and set the host thread
+    count of the full-size kernels (0 = all cores). Returns the thread count in effect."""
     global _LIB, LIB_PATH
-    build(native=True, force=True)  # the .so may have travelled from another CPU: always rebuild on this box
-    LIB_PATH = NATIVE_LIB_PATH
+    LIB_PATH = build(native=True)
     _LIB = None
     return set_threads(threads)
 

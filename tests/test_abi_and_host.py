@@ -31,14 +31,14 @@ def test_header_symbols_are_exported_and_bound():
     assert b"b200ba" in lib.b200ba_version()
 
 
-def test_struct_layouts_match_header():
+def test_struct_layouts_match_header(tmp_path):
     """sizeof of the ctypes mirrors equals what the C compiler lays out."""
     src = r'''
 #include <stdio.h>
 #include "b200ba.h"
 int main(){printf("%zu %zu %zu %zu %zu %zu %zu\n", sizeof(b200ba_camera), sizeof(b200ba_problem), sizeof(b200ba_state),
  sizeof(b200ba_options), sizeof(b200ba_report), sizeof(b200ba_timings), sizeof(b200ba_fit_report));return 0;}'''
-    exe = "/tmp/_b200ba_sizes"
+    exe = str(tmp_path / "b200ba_sizes")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.join(ROOT, "include"), "-o", exe], input=src.encode(), check=True)
     sizes = [int(v) for v in subprocess.check_output([exe]).split()]
     mine = [C.sizeof(t) for t in (cabi.Camera, cabi.Problem, cabi.State, cabi.Options, cabi.Report, cabi.Timings, cabi.FitReport)]

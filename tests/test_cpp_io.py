@@ -11,10 +11,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
-def exe():
+def exe(tmp_path_factory):
     from camera_calibration_b200 import build
     build.build()
-    path = "/tmp/b200ba_io_example"
+    path = str(tmp_path_factory.mktemp("io_example") / "b200ba_io_example")
     lib_dir = os.path.join(ROOT, "camera_calibration_b200", "csrc")
     subprocess.check_call(["g++", "-std=c++17", "-O1", "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"),
                            os.path.join(ROOT, "tests", "io_example.cc"), "-o", path, "-L", lib_dir, "-lb200ba",

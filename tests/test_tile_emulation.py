@@ -9,8 +9,8 @@ import subprocess
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_tile_program_on_the_host():
-    exe = "/tmp/b200ba_tile_emulation"
+def test_tile_program_on_the_host(tmp_path):
+    exe = str(tmp_path / "b200ba_tile_emulation")
     subprocess.check_call(["g++", "-std=c++17", "-O1", "-Wall", "-Wno-unknown-pragmas",
                            os.path.join(ROOT, "tests", "tile_emulation.cc"), "-o", exe])
     r = subprocess.run([exe], capture_output=True, text=True)
